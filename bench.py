@@ -55,7 +55,14 @@ def parse():
                     "`ncu --profile-from-start off --metrics dram__bytes_read.sum,dram__bytes_write.sum`: DRAM bytes per step)")
     ap.add_argument("--cfg", default=None, help="other config to exercise (P2B_Car.yaml, M2_track_kitti.yaml, ...): a parity / "
                     "plumbing run of BASELINE.json configs[2..4], NOT the headline metric")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last device-timed step computed (loss, gradients, updated "
+                         "parameters, BatchNorm running statistics) as DIR/<name>.npy; that step starts from the model's initial "
+                         "state, so that two runs or builds can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.track or args.sampler):
+        ap.error("--dump-outputs writes the training step's outputs; it does not apply to --impl reference, --track or --sampler")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------- clocks
@@ -565,6 +572,38 @@ def kernel_table(eng, batches, path, steps=3):
             f.write(f"{100 * us / total:7.2f}% {us / steps / 1e3:9.3f} {n / steps:8.1f}  {name[:150]}\n")
 
 
+def train_state(eng):
+    """What a training step reads besides its batch: parameters, Adam moments and step counter, BatchNorm buffers."""
+    return [eng.flat.flat, eng.opt.exp_avg, eng.opt.exp_avg_sq, eng.opt.state, *eng.model.buffers()]
+
+
+def step_outputs(eng, loss):
+    """Device copies of what a training step computes: the loss `TrainStep.step` returns, the gradient of every parameter and
+    the parameters after the Adam update (each one flat float32 array in `model.parameters()` order, as the engine keeps
+    them), and the BatchNorm running statistics the step leaves in the model.
+    The backward scatters with float atomics, so gradients repeat from run to run only to rounding; compare with a tolerance
+    scaled to each array (a few gradients are 0 in exact arithmetic, e.g. of a bias feeding BatchNorm, and hold only rounding,
+    which Adam's lr * g / (|g| + eps) carries into the parameters as about lr / eps times that rounding).  Two runs of
+    BAT_Car.yaml on one B200 (1,000 W): loss and BatchNorm statistics bitwise equal; gradients 6.0e-7 apart normwise (at
+    most 2.2e-6 in an element, largest |g| 0.93); parameters 9.0e-7 normwise (at most 3.3e-5 in an element, largest 3.2)."""
+    out = {"loss": loss.reshape(1), "gradients": eng.flat.grad, "parameters": eng.flat.flat}
+    for k, b in eng.model.named_buffers():
+        out["buffer." + k] = b
+    return {k: v.detach().clone() for k, v in out.items()}
+
+
+def write_outputs(outputs, out_dir, limit_bytes=64 << 20):
+    """DIR/<name>.npy for every output, float32 (integer counters as float64)."""
+    import numpy as np
+    arrays = {k: v.cpu().numpy() for k, v in outputs.items()}
+    arrays = {k: v.astype(np.float32 if v.dtype.kind == "f" else np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= limit_bytes, f"--dump-outputs: {total} bytes exceed the {limit_bytes}-byte limit"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def run_ours(args):
     from open3dsot_b200 import ddp, ops, runtime
     from open3dsot_b200.config import load_config
@@ -593,6 +632,10 @@ def run_ours(args):
     net = get_model(cfg.net_model)(cfg).to(dev).train()
     from open3dsot_b200.engine import TrainStep
     eng = TrainStep(net, lr=cfg.lr, weight_decay=cfg.wd, use_graph=not args.no_graph, warmup=2)
+    # --dump-outputs: the last device-timed step restarts from this initial state (restored outside its timed window).  The
+    # kernels' float atomics round differently from run to run and training amplifies that over the ~30 earlier steps, so
+    # only a step from a known state can be compared between runs and builds.
+    initial_state = [t.clone() for t in train_state(eng)] if args.dump_outputs else None
 
     # distinct host batches (pinned), one device-resident copy of each
     n_batches = 4
@@ -642,12 +685,16 @@ def run_ours(args):
     barrier()
     t_wall0 = time.perf_counter()
     for i in range(args.steps):
+        if initial_state is not None and i == args.steps - 1:
+            for t, t0 in zip(train_state(eng), initial_state):  # not timed; before the flush, so this step starts cold too
+                t.copy_(t0)
         flush.fill_(float(i))                                   # evict L2; not timed
         evs[i][0].record()
-        eng.step(resident[i % n_batches])
+        loss = eng.step(resident[i % n_batches])
         evs[i][1].record()
     barrier()
     wall = time.perf_counter() - t_wall0
+    outputs = step_outputs(eng, loss) if args.dump_outputs else None
     launches = launches_per_step * args.steps
     dev_ms = sum(a.elapsed_time(b) for a, b in evs)
     t = torch.tensor([dev_ms], dtype=torch.float64, device=dev)
@@ -699,6 +746,8 @@ def run_ours(args):
     if rank != 0:
         _shutdown(eng, world)
         return
+    if outputs is not None:
+        write_outputs(outputs, args.dump_outputs)
     if args.kernel_table:
         kernel_table(eng, resident, args.kernel_table)
     roof = roofline_probe(dev, args.batch)

@@ -237,25 +237,74 @@ def gen_m2track(out):
     out["m2_eval_boxes"] = np_(ep["estimation_boxes"])
 
 
-def gen_checkpoint_eval(out):
-    """SURVEY.md §8f rank 1: the reference's shipped `pretrained_models/bat_kitti_car.ckpt` through the reference's own BAT in
-    eval mode on a fixed synthetic pair -> outputs (committed) + the state dict as a plain npz under tests/golden/_ckpt/
-    (git-ignored: trained weights are not source; the GPU box receives the file with the working tree)."""
+def gen_checkpoint_eval():
+    """SURVEY.md §8f rank 1: the trained weights of the reference's shipped `pretrained_models/bat_kitti_car.ckpt` (6 MB of
+    float32), stored as 4-bit codes per output channel with BatchNorm statistics and biases exact (tests/_params.py
+    `pack_state_4bit`), and what the reference's own BAT computes in eval mode with exactly those weights on a fixed
+    synthetic pair -> bat_kitti_car_q4.npz (weights under their state-dict keys, outputs under 'out:<name>')."""
     from models import get_model
     from open3dsot_b200.checkpoint import load_lightning_checkpoint
+    from _params import pack_state_4bit, unpack_state_4bit
     ck = load_lightning_checkpoint(os.path.join(REF, "pretrained_models", "bat_kitti_car.ckpt"))
     cfg = EasyDict(load_yaml(os.path.join(ROOT, "cfgs", "BAT_Car.yaml")))
     net = get_model(cfg.net_model)(cfg)
-    missing = net.load_state_dict(ck["state_dict"], strict=False)
-    assert not [k for k in missing.missing_keys if not k.split(".")[0] in ("prec", "success")], missing
+    packed = pack_state_4bit({k: v for k, v in ck["state_dict"].items() if k in net.state_dict()})
+    net.load_state_dict(unpack_state_4bit(packed), strict=True)
     net.eval()
     batch = synthetic_siamese_batch(2, 512, 1024, seed=4242, box_aware=True)
     with torch.no_grad():
         ep = net({k: v.clone() for k, v in batch.items()})
     for k in ("estimation_boxes", "estimation_cla", "vote_xyz", "center_xyz", "sample_idxs", "pred_search_bc"):
-        out[f"ckpt_bat_car_{k}"] = np_(ep[k])
-    os.makedirs(os.path.join(HERE, "_ckpt"), exist_ok=True)
-    np.savez(os.path.join(HERE, "_ckpt", "bat_kitti_car_state.npz"), **{k: np_(v) for k, v in ck["state_dict"].items()})
+        packed[f"out:{k}"] = np_(ep[k])
+    np.savez_compressed(os.path.join(HERE, "bat_kitti_car_q4.npz"), **packed)
+
+
+def _with_tensors(obj, fn):
+    """Apply `fn` to every tensor inside nested dicts / lists / tuples, in place where the container allows."""
+    if isinstance(obj, torch.Tensor):
+        return fn(obj)
+    if isinstance(obj, dict):
+        for k in list(obj):
+            obj[k] = _with_tensors(obj[k], fn)
+    elif isinstance(obj, list):
+        obj[:] = [_with_tensors(x, fn) for x in obj]
+    elif isinstance(obj, tuple):
+        obj = type(obj)(_with_tensors(x, fn) for x in obj)
+    return obj
+
+
+def gen_checkpoint_skeletons():
+    """The reference's shipped checkpoints (18-27 MB each) cut down for tests/test_checkpoint_compat.py: every tensor keeps
+    its first value, viewed at its full shape with zero strides, so the file has the original's format (legacy pickle or
+    zip), top-level keys, state-dict key order, shapes and dtypes, optimizer-state layout, hyper-parameters (pickled as
+    `easydict.EasyDict`) and Lightning bookkeeping (the `ModelCheckpoint` class as a callbacks key) in a few KiB."""
+    import zipfile
+    from open3dsot_b200.checkpoint import load_lightning_checkpoint
+    os.makedirs(os.path.join(HERE, "checkpoints"), exist_ok=True)
+    for name in ("bat_kitti_car.ckpt", "bat_kitti_pedestrian.ckpt", "mmtrack_kitti_car.ckpt"):
+        src = os.path.join(REF, "pretrained_models", name)
+        ck = load_lightning_checkpoint(src)
+        _with_tensors(ck, lambda t: t.reshape(-1)[:1].clone().reshape([1] * t.dim()).expand(t.shape) if t.numel() else t)
+        # globals the restricted unpickler turned into placeholders, and our EasyDict, are written under their original names
+        names = {k.__module__: k for k in ck.get("callbacks", {}) if isinstance(k, type)}
+        saved = {m: sys.modules.get(m) for m in ["easydict"] + [".".join(p.split(".")[:i + 1]) for p in names
+                                                                for i in range(p.count(".") + 1)]}
+        for m in saved:
+            sys.modules[m] = types.ModuleType(m)
+        for m, cls in names.items():
+            setattr(sys.modules[m], cls.__name__, cls)
+        old = (EasyDict.__module__, EasyDict.__qualname__)
+        EasyDict.__module__, EasyDict.__qualname__ = "easydict", "EasyDict"
+        sys.modules["easydict"].EasyDict = EasyDict
+        try:
+            torch.save(ck, os.path.join(HERE, "checkpoints", name), _use_new_zipfile_serialization=zipfile.is_zipfile(src))
+        finally:
+            EasyDict.__module__, EasyDict.__qualname__ = old
+            for m, mod in saved.items():
+                if mod is None:
+                    sys.modules.pop(m, None)
+                else:
+                    sys.modules[m] = mod
 
 
 def main():
@@ -269,9 +318,10 @@ def main():
     gen_model("bat", "BAT_Car.yaml", 2, 256, 512, models, seed=21)
     gen_model("p2b", "P2B_Car.yaml", 2, 256, 512, models, seed=22)   # BASELINE.json configs[0] shape; B=2 (B=1 is a degenerate BatchNorm case)
     gen_m2track(models)
-    gen_checkpoint_eval(models)
     np.savez_compressed(os.path.join(HERE, "ref_models.npz"), **models)
-    for f in ("ref_modules.npz", "ref_models.npz"):
+    gen_checkpoint_eval()
+    gen_checkpoint_skeletons()
+    for f in ("ref_modules.npz", "ref_models.npz", "bat_kitti_car_q4.npz"):
         print(f, os.path.getsize(os.path.join(HERE, f)) // 1024, "KiB")
 
 

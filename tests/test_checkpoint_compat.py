@@ -1,5 +1,7 @@
 """Drop-in check of the checkpoint surface (SURVEY.md §8f rank 1): the reference's shipped BAT / M2-Track checkpoints
-load, key for key, into our modules.  Runs only where /root/reference exists (the authoring container)."""
+load, key for key, into our modules.  The files under tests/golden/checkpoints/ are those checkpoints cut down by
+tests/golden/make_golden.py: the original format, keys, shapes, hyper-parameters and Lightning bookkeeping, with every
+tensor reduced to its first value (stride-0 views), since the originals are 18-27 MB each."""
 import os
 
 import pytest
@@ -10,8 +12,7 @@ from open3dsot_b200.config import load_config
 from open3dsot_b200.models import get_model
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CKPT_DIR = "/root/reference/pretrained_models"
-pytestmark = pytest.mark.skipif(not os.path.isdir(CKPT_DIR), reason="reference checkpoints not present on this box")
+CKPT_DIR = os.path.join(ROOT, "tests", "golden", "checkpoints")
 
 
 @pytest.mark.parametrize("ckpt,cfg_file", [("bat_kitti_car.ckpt", "BAT_Car.yaml"),
