@@ -5,8 +5,10 @@
  *   - every pointer is a DEVICE pointer unless its name ends in `_host`; the caller owns all buffers,
  *     including scratch and pre-zeroed gradient outputs — nothing is allocated inside;
  *   - float = IEEE fp32, indices = int32, tensors dense row-major in the shape given in the comment;
- *   - `stream` is a cudaStream_t passed as void*; kernels are only enqueued (no synchronisation, no
- *     host-side state), so every entry point may be captured into a CUDA graph;
+ *   - `stream` is a cudaStream_t passed as void*; kernels are only enqueued (no synchronisation), so
+ *     every entry point may be captured into a CUDA graph;
+ *   - no host-side state: what an entry point does depends on its arguments only.  The one exception
+ *     is the process-wide force_mt switch of o3d_debug_set(), the library's only mutable global;
  *   - return value 0 = ok, <0 = argument / CUDA error; o3d_last_error() gives the text (thread-local);
  *   - no torch types anywhere.
  *
@@ -192,8 +194,9 @@ int o3d_dense_bwd_prep(const float* dout, int ldd, const float* out, int ldo, co
  * forward:  rows = Cout, K = Cin   (w = the padded conv weight)
  * dgrad  :  rows = Cin,  K = Cout  (w = its transpose)                                                */
 long long o3d_pw_tc_wtile_bytes(int rows, int K);
-void o3d_pw_tc_set_reverse(int rev);              /* next o3d_pw_*_tc launch of this thread walks the position tiles backwards */
-void o3d_debug_set(int tc_debug, int force_mt);   /* profiling experiments only (results invalid when non-zero) */
+/* Measurement switch, process-wide and not synchronised: force_mt = 1 makes every tensor-core GEMM take one 128-channel
+ * tile per CTA.  tc_debug must be 0; anything but (0, 0) and (0, 1) returns O3D_ERR_ARG and changes nothing.        */
+int o3d_debug_set(int tc_debug, int force_mt);
 int o3d_pw_tc_pretile(const float* w, int ldw, int rows, int K, void* wtiles, void* stream);
 int o3d_pw_fwd_tc(const float* x, int ldx, const float* in_scale, const float* in_shift, int in_relu, const void* wtiles,
                   const float* bias, int P, int K, int N, float* y, int ldy, double* sum, double* sumsq, int S,
@@ -247,7 +250,8 @@ typedef struct o3d_stack_t {
     int K0;         /* input row length (multiple of 4, zero padded)                             */
     int S;          /* pooling group size over consecutive positions (0 = dense output)          */
     int training;   /* BatchNorm uses batch statistics and updates the running ones              */
-    int use_tc;     /* allow the tcgen05 3xTF32 kernels where the shape qualifies                */
+    int use_tc;     /* tcgen05 3xTF32 kernels where the shape qualifies: bit 0 forward + dgrad, bit 1 wgrad;
+                       other bits are rejected                                                   */
     int xyz_first;  /* layer-0 weight columns are [xyz(3) | features(c0)], input rows [features | dx dy dz 0] */
     int c0;         /* real feature channels of layer 0 when xyz_first                           */
     int dx_cols;    /* backward: only the first dx_cols input columns need a gradient (0 = all K0) */
@@ -302,29 +306,10 @@ int o3d_sa_fused_forward(const o3d_stack_t* d, const void* block, const float* x
  * o3d_lift_stats : gidx[p] = global Z row of position p; sum / sumsq (nullable) += per-channel batch statistics of Y0;
  *                  y0 (nullable) receives Y0 itself [P, C0] (the CUDA-core fallback reads it as an ordinary activation).
  * o3d_lift_scatter: dY0 = a*g + b + cc*Y0 (a == NULL: dY0 = g) scattered into lf->d_z / d_cc / d_s / d_u (see o3d_lift_t);
- *                  y0 NULL = re-gather Y0 from Z.
- * o3d_pw_*_tc_lift: the tensor-core GEMMs of the layer AFTER the lifted one, reading Y0 through gidx (never stored).
- *                  wgrad: part != NULL selects the wide-tile split-K kernel (deterministic), NULL the 128x128 RED kernel.   */
+ *                  y0 NULL = re-gather Y0 from Z.                                                                          */
 int o3d_lift_stats(const o3d_lift_t* lf, int P, int C0, int32_t* gidx, float* y0, double* sum, double* sumsq, void* stream);
 int o3d_lift_scatter(const o3d_lift_t* lf, int P, int C0, const int32_t* gidx, const float* y0, const float* g, int ldg,
                      const float* a, const float* b, const float* cc, void* stream);
-int o3d_pw_fwd_tc_lift(const o3d_lift_t* lf, const int32_t* gidx, const float* in_scale, const float* in_shift, int in_relu,
-                       const void* wtiles, const float* bias, int P, int K, int N, float* y, int ldy, double* sum,
-                       double* sumsq, int S, float* ymax, float* ymin, int32_t* arg, int ldp, void* stream);
-int o3d_pw_dgrad_tc_lift(const float* g, int ldg, const float* y, int ldy, const float* a, const float* b, const float* cc,
-                         const float* dpool, const int32_t* sel, int S, int ldp, const void* wtiles_t, int P, int Cout,
-                         int Cin, float* out, int ldo, const o3d_lift_t* lf, const int32_t* gidx, const float* pscale,
-                         const float* pshift, int prelu, double* s1, double* s2y, void* stream);
-int o3d_pw_wgrad_tc_lift(const float* g, int ldg, const float* y, int ldy, const float* a, const float* b, const float* cc,
-                         const float* dpool, const int32_t* sel, int S, int ldp, const o3d_lift_t* lf, const int32_t* gidx,
-                         const float* in_scale, const float* in_shift, int in_relu, int P, int Cout, int Cin, float* dw,
-                         int lddw, float* part, long long part_floats, void* stream);
-
-/* wgrad on the tensor core (MN-major SWIZZLE_128B operands, split over positions, fp32 RED into dw). */
-int o3d_pw_wgrad_tc(const float* g, int ldg, const float* y, int ldy, const float* a, const float* b, const float* cc,
-                    const float* dpool, const int32_t* sel, int S, int ldp, const float* x, int ldx,
-                    const float* in_scale, const float* in_shift, int in_relu, int P, int Cout, int Cin, float* dw,
-                    int lddw, void* stream);
 
 /* wgrad, wide tiles (up to 256 x 256 of dW per CTA, all of TMEM), split over positions; the per-split partial tiles go
  * to `part` (o3d_pw_wgrad_tc2_workspace_floats() floats) and a second kernel adds their sum into dw.              */

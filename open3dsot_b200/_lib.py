@@ -50,12 +50,10 @@ PROTOTYPES = {
     "o3d_dense_bwd_prep": [_p, _i, _p, _i, _p, _i, _i, _i, _i, _p, _i, _p, _p, _p],
     "o3d_pw_tc_wtile_bytes": [_i, _i],
     "o3d_debug_set": [_i, _i],
-    "o3d_pw_tc_set_reverse": [_i],
     "o3d_pw_tc_pretile": [_p, _i, _i, _i, _p, _p],
     "o3d_pw_fwd_tc": [_p, _i, _p, _p, _i, _p, _p, _i, _i, _i, _p, _i, _p, _p, _i, _p, _p, _p, _i, _p],
     "o3d_pw_dgrad_tc": [_p, _i, _p, _i, _p, _p, _p, _p, _p, _i, _i, _p, _i, _i, _i, _p, _i, _p, _i, _p, _p, _i, _p, _p,
                         _p],
-    "o3d_pw_wgrad_tc": [_p, _i, _p, _i, _p, _p, _p, _p, _p, _i, _i, _p, _i, _p, _p, _i, _i, _i, _i, _p, _i, _p],
     "o3d_pw_wgrad_tc2_workspace_floats": [],
     "o3d_pw_wgrad_tc2": [_p, _i, _p, _i, _p, _p, _p, _p, _p, _i, _i, _p, _i, _p, _p, _i, _i, _i, _i, _p, _i, _p,
                          ctypes.c_longlong, _p],
@@ -64,11 +62,6 @@ PROTOTYPES = {
     "o3d_resample": [_p, _p, _p, _p, _i, _i, _i, _p, _p, _p, _p, _p],
     "o3d_lift_stats": [_p, _i, _i, _p, _p, _p, _p, _p],
     "o3d_lift_scatter": [_p, _i, _i, _p, _p, _p, _i, _p, _p, _p, _p],
-    "o3d_pw_fwd_tc_lift": [_p, _p, _p, _p, _i, _p, _p, _i, _i, _i, _p, _i, _p, _p, _i, _p, _p, _p, _i, _p],
-    "o3d_pw_dgrad_tc_lift": [_p, _i, _p, _i, _p, _p, _p, _p, _p, _i, _i, _p, _i, _i, _i, _p, _i, _p, _p, _p, _p, _i, _p,
-                             _p, _p],
-    "o3d_pw_wgrad_tc_lift": [_p, _i, _p, _i, _p, _p, _p, _p, _p, _i, _i, _p, _p, _p, _p, _i, _i, _i, _i, _p, _i, _p,
-                             ctypes.c_longlong, _p],
     "o3d_stack_workspace_bytes": [_p, _i],
     "o3d_stack_prepared_bytes": [_p],
     "o3d_stack_prepare": [_p, _p, _p],
@@ -80,8 +73,7 @@ PROTOTYPES = {
 }
 _RESTYPE = {"o3d_last_error": ctypes.c_char_p, "o3d_pw_tc_wtile_bytes": ctypes.c_longlong,
             "o3d_stack_workspace_bytes": ctypes.c_longlong, "o3d_stack_prepared_bytes": ctypes.c_longlong,
-            "o3d_sa_fused_prepared_bytes": ctypes.c_longlong, "o3d_debug_set": None, "o3d_pw_tc_set_reverse": None,
-            "o3d_pw_wgrad_tc2_workspace_floats": ctypes.c_longlong}
+            "o3d_sa_fused_prepared_bytes": ctypes.c_longlong, "o3d_pw_wgrad_tc2_workspace_floats": ctypes.c_longlong}
 
 MAX_LAYERS = 8
 _I8, _F8, _P8 = ctypes.c_int * MAX_LAYERS, ctypes.c_float * MAX_LAYERS, ctypes.c_void_p * MAX_LAYERS

@@ -133,7 +133,5 @@ __device__ __forceinline__ uint32_t o3d_lanemask_lt() {
     asm("mov.u32 %0, %%lanemask_lt;" : "=r"(m));
     return m;
 }
-// debug switch (o3d_debug_set bit 7): few-column wgrads go through the tiled CUDA-core kernel instead of the streaming one
-extern int o3d_g_no_skinny;
 
 #endif

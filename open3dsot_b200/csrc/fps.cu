@@ -22,8 +22,6 @@
 #include "common.cuh"
 #include "../../include/o3d_b200.h"
 
-int o3d_g_fps_wide = 0;     // experiment switch (o3d_debug_set bit 10): twice the threads, half the points per thread
-
 namespace {
 
 struct FpsParams {
@@ -150,14 +148,14 @@ extern "C" int o3d_fps(const float* xyz, int B, int N, int npoint, int32_t* idx,
     // more warps shortens the per-thread chain (the second-level reduction handles up to 32 warps in one step)
     if (N <= 128) return launch_fps<128, 1>(xyz, B, idx, prm, st);
     if (N <= 256) return launch_fps<128, 2>(xyz, B, idx, prm, st);
-    // measured, N = 1024 -> 512 (cycles per iteration at 1965 MHz): 128 x 8: 1,170 (round 1) | 256 x 4: 660 | 512 x 2: 427 | 1024 x 1: see
-    // o3d_debug_set bit 10;  N = 512 -> 256: 256 x 2: 330 | 512 x 1: 338.  Tried and dropped: a (x, y, z, index) float4 decode table
+    // measured, N = 1024 -> 512 (cycles per iteration at 1965 MHz): 128 x 8: 1,170 (round 1) | 256 x 4: 660 | 512 x 2: 427 | 1024 x 1:
+    // tried, slower; no time recorded;  N = 512 -> 256: 256 x 2: 330 | 512 x 1: 338.  Tried and dropped: a (x, y, z, index) float4 decode table
     // (one 16-byte LDS instead of the index lookup + three dependent coordinate loads): 512 x 2 went from 107 us to 145 us;
     // the block-level arg-max as one 64-bit shared-memory atomicMax of (key << 32 | ~priority) per warp instead of three of the
     // four warp reductions: 64-bit shared atomics compile to an LDS + ATOMS.CAS retry loop, and resampled clouds are full of
     // exact duplicates (ties -> many lanes enter it): 110 -> 233 us.
     if (N <= 512) return launch_fps<256, 2>(xyz, B, idx, prm, st);
-    if (N <= 1024) return o3d_g_fps_wide ? launch_fps<1024, 1>(xyz, B, idx, prm, st) : launch_fps<512, 2>(xyz, B, idx, prm, st);
+    if (N <= 1024) return launch_fps<512, 2>(xyz, B, idx, prm, st);
     if (N <= 2048) return launch_fps<256, 8>(xyz, B, idx, prm, st);
     if (N <= 4096) return launch_fps<256, 16>(xyz, B, idx, prm, st);
     if (N <= 8192) return launch_fps<512, 16>(xyz, B, idx, prm, st);

@@ -887,8 +887,6 @@ inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 
 
 }  // namespace
 
-int o3d_g_no_skinny = 0;
-
 // ============================================================================================================
 extern "C" int o3d_pw_fwd(const float* x, int ldx, const float* in_scale, const float* in_shift, int in_relu,
                           const float* wt, int ldw, const float* bias, int P, int K, int N, float* y, int ldy,
@@ -908,7 +906,7 @@ extern "C" int o3d_pw_fwd(const float* x, int ldx, const float* in_scale, const 
     ActIn ain{x, ldx, in_scale, in_shift, in_relu};
     FwdEpi ep{y, ldy, bias, sum, sumsq, S, ymax, ymin, arg, ldp};
     cudaStream_t st = (cudaStream_t)stream;
-    if (K <= 8 && S == 0 && P >= 4096 && !o3d_g_no_skinny) {
+    if (K <= 8 && S == 0 && P >= 4096) {
         if (K <= 4) return launch_fwd_skinny<1>(ain, wt, ldw, P, K, Nw, ep, st);
         return launch_fwd_skinny<2>(ain, wt, ldw, P, K, Nw, ep, st);
     }
@@ -970,7 +968,7 @@ extern "C" int o3d_pw_wgrad(const float* g, int ldg, const float* y, int ldy, co
     DyIn din = make_dy(g, ldg, y, ldy, a, b, cc, dpool, sel, S, ldp);
     ActIn ain{x, ldx, in_scale, in_shift, in_relu};
     cudaStream_t st = (cudaStream_t)stream;
-    if (Cin <= 12 && P >= 4096 && !o3d_g_no_skinny) {
+    if (Cin <= 12 && P >= 4096) {
         if (Cin <= 4) return launch_wgrad_skinny<1, 4>(din, ain, P, Cout, Cin, dw, lddw, st);
         if (Cin <= 8) return launch_wgrad_skinny<2, 2>(din, ain, P, Cout, Cin, dw, lddw, st);
         return launch_wgrad_skinny<3, 2>(din, ain, P, Cout, Cin, dw, lddw, st);

@@ -24,16 +24,14 @@
 //   warps 2,3,12-17  operand producers (256 threads, 4 neighbouring rows each): coalesced 16-byte loads issued one
 //                 k-block ahead ("raw-first"), transform, hi/lo split, 128B-swizzled st.shared, fence.proxy.async, arrive
 // Shared memory: MT = 1: 3 stages x (W 32K | X 32K) = 192 KB;  MT = 2: 2 stages x (W 64K | X 32K) = 192 KB; K-major
-// SWIZZLE_128B tiles.  The wgrad kernels further down have their own role tables.
+// SWIZZLE_128B tiles.  The wgrad kernel further down has its own role table.
 #include "common.cuh"
 #include "lift.cuh"
+#include "pwmlp_tc.cuh"
 #include "tc_ptx.cuh"
 #include "../../include/o3d_b200.h"
 
 namespace {
-
-constexpr int TC_STAGES = 3;
-constexpr int STAGE_BYTES = 4 * TILE_BYTES;            // Whi | Wlo | Xhi | Xlo
 
 // ---- operand descriptions (same semantics as ActIn / DyIn in pwmlp.cu) --------------------------------------
 // `prep(k)` fetches the per-channel coefficients of the thread's 4 channels once per k-block; `row(p)` then costs one
@@ -162,7 +160,6 @@ struct TcDy {
     const float* g; int ldg; const float* y; int ldy; const float* a; const float* b; const float* cc;
     const float* dpool; const int32_t* sel; int S; int ldp;
     int sh;   // S == 1 << sh (pooling group sizes are powers of two on this path)
-    int dbg;  // profiling experiments: 256 = no sel / dpool loads, 512 = no y load
     struct Coef { float4 a, b, c; bool on; };
     // raw operand rows of one thread for one k-block: rows p0 + i * stride, i < R (R >= 2).
     // Pooled gradient: when all R rows fall into one pooling group — the usual case, a thread's rows are neighbours — the
@@ -188,13 +185,9 @@ struct TcDy {
             if (R >= 2 && (pf >> sh) == (pl >> sh)) {   // the two tables live in g[0], g[1]
                 bt.shared = true;
                 const size_t go = (size_t)(pf >> sh) * ldp + kk;
-                if (!(dbg & 256)) {
-                    bt.g[0] = ld4g(dpool + go);
-                    const int4 sl = __ldg(reinterpret_cast<const int4*>(sel + go));
-                    bt.g[R >= 2 ? 1 : 0] = make_float4(__int_as_float(sl.x), __int_as_float(sl.y), __int_as_float(sl.z), __int_as_float(sl.w));
-                } else {
-                    bt.g[0] = bt.g[R >= 2 ? 1 : 0] = make_float4(0.f, 0.f, 0.f, 0.f);
-                }
+                bt.g[0] = ld4g(dpool + go);
+                const int4 sl = __ldg(reinterpret_cast<const int4*>(sel + go));
+                bt.g[R >= 2 ? 1 : 0] = make_float4(__int_as_float(sl.x), __int_as_float(sl.y), __int_as_float(sl.z), __int_as_float(sl.w));
             } else {
 #pragma unroll
                 for (int i = 0; i < R; ++i) {
@@ -216,7 +209,7 @@ struct TcDy {
 #pragma unroll
         for (int i = 0; i < R; ++i) {
             const int p = p0 + i * stride;
-            bt.y[i] = (a && !(dbg & 512)) ? ld4g(y + (size_t)(p < P ? p : P - 1) * ldy + kk) : make_float4(0.f, 0.f, 0.f, 0.f);
+            bt.y[i] = a ? ld4g(y + (size_t)(p < P ? p : P - 1) * ldy + kk) : make_float4(0.f, 0.f, 0.f, 0.f);
         }
     }
     template <int R>
@@ -453,11 +446,9 @@ template <int MT> struct TcCfg {
 };
 constexpr int TC2_THREADS = 576;   // 18 warps: 0 MMA | 1 weights | 2,3,12-17 producers | 4-11 epilogue
 
-// dbg (profiling experiments only; results are wrong when set): 1 = stream weights for the first tile only,
-// 2 = producers skip the global loads, 4 = epilogue skips its global stores / loads
 template <int MT, class BLoad, class Epi>
 __global__ void __launch_bounds__(TC2_THREADS, 1)
-    pw_tc_kernel(BLoad bl, const uint8_t* __restrict__ wtiles, int P, int K, int Nw, int nkb, Epi epi, int dbg, int rev) {
+    pw_tc_kernel(BLoad bl, const uint8_t* __restrict__ wtiles, int P, int K, int Nw, int nkb, Epi epi, int rev) {
     using C = TcCfg<MT>;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -529,24 +520,20 @@ __global__ void __launch_bounds__(TC2_THREADS, 1)
         // ===================================================== weight-tile streamer (bulk copy engine)
         if (lane == 0) {
             int stage = 0, phase = 0;
-            if (!(dbg & 8) && (int)blockIdx.x < n_ptiles) {
+            if ((int)blockIdx.x < n_ptiles) {
                 bl.prefetch_rows(tile_of(blockIdx.x) * TC_N, TC_N, P);
             }
             for (int t = blockIdx.x; t < n_ptiles; t += gridDim.x) {
-                if (!(dbg & 8) && t + (int)gridDim.x < n_ptiles) {
+                if (t + (int)gridDim.x < n_ptiles) {
                     bl.prefetch_rows(tile_of(t + (int)gridDim.x) * TC_N, TC_N, P);   // next tile of this CTA -> L2
                 }
                 for (int kb = 0; kb < nkb; ++kb) {
                     o3d_mbar_wait(empty + stage, phase ^ 1);
-                    if ((dbg & 1) && t != (int)blockIdx.x) {
-                        o3d_mbar_arrive(full + stage);
-                    } else {
-                        o3d_mbar_expect_tx(full + stage, MT * 2 * TILE_BYTES);
+                    o3d_mbar_expect_tx(full + stage, MT * 2 * TILE_BYTES);
 #pragma unroll
-                        for (int m = 0; m < MT; ++m)
-                            o3d_bulk_g2s(smem + stage * C::STAGE_BYTES_ + 2 * m * TILE_BYTES,
-                                         wtiles + ((size_t)(mt0 + m) * nkb + kb) * (2 * TILE_BYTES), 2 * TILE_BYTES, full + stage);
-                    }
+                    for (int m = 0; m < MT; ++m)
+                        o3d_bulk_g2s(smem + stage * C::STAGE_BYTES_ + 2 * m * TILE_BYTES,
+                                     wtiles + ((size_t)(mt0 + m) * nkb + kb) * (2 * TILE_BYTES), 2 * TILE_BYTES, full + stage);
                     if (++stage == C::STAGES) { stage = 0; phase ^= 1; }
                 }
             }
@@ -559,7 +546,6 @@ __global__ void __launch_bounds__(TC2_THREADS, 1)
         const int cg0 = MT == 2 ? 0 : grp * 4, cg1 = MT == 2 ? 8 : grp * 4 + 4;   // 16-column groups to handle
         const int ch = (mt0 + m) * TC_M + q * 32 + lane;
         epi.begin(ch, Nw);
-        const int Nw_e = (dbg & 4) ? 0 : Nw;          // dbg: ch >= Nw_e -> the epilogue body is skipped
         int acc = 0, aphase = 0;
         int32_t* gsm = reinterpret_cast<int32_t*>(smem + C::STAGES * C::STAGE_BYTES_ + 256);   // [2][TC_N] row indices
         float4* ssm = reinterpret_cast<float4*>(smem + C::STAGES * C::STAGE_BYTES_ + 256 + 1024);   // [2][TC_N] per-position scalars
@@ -578,7 +564,7 @@ __global__ void __launch_bounds__(TC2_THREADS, 1)
                     epi.set_tile(gsm + acc * TC_N, ssm + acc * TC_N);
                 }
             }
-            epi.prefetch(ch, Nw_e, pt0 + cg0 * 16, P);
+            epi.prefetch(ch, Nw, pt0 + cg0 * 16, P);
             o3d_mbar_wait(tfull + acc, aphase);
             tc_fence_after();
             const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)((acc * MT + m) * TC_N);
@@ -586,8 +572,8 @@ __global__ void __launch_bounds__(TC2_THREADS, 1)
             for (int cg = cg0; cg < cg1; ++cg) {
                 uint32_t r[16];
                 tmem_ld16(taddr + cg * 16, r);
-                epi.group(r, ch, Nw_e, pt0 + cg * 16, P);
-                if (cg + 1 < cg1) epi.prefetch(ch, Nw_e, pt0 + (cg + 1) * 16, P);
+                epi.group(r, ch, Nw, pt0 + cg * 16, P);
+                if (cg + 1 < cg1) epi.prefetch(ch, Nw, pt0 + (cg + 1) * 16, P);
             }
             tc_fence_before();
             o3d_mbar_arrive(tempty + acc);
@@ -604,7 +590,6 @@ __global__ void __launch_bounds__(TC2_THREADS, 1)
         const int chunk = pt & 7;                         // 16-byte chunk (4 channels) inside the 128-byte row
         const int row0 = (pt >> 3) * 4;                   // 4 neighbouring rows row0 + i, i < 4 (one pooling group)
         int stage = 0, phase = 0;
-        if (dbg & 2) P = 0;                               // dbg: nothing is loaded
         // The (tile, k-block) nest is walked as one flat sequence of items so that the raw loads of the items ahead — also
         // when they belong to the next position tile — are in flight while the current one is being stored.  A loader with
         // DEPTH == 2 (the forward operand: 16 raw registers per item) keeps two items in flight per thread: one k-block
@@ -622,7 +607,7 @@ __global__ void __launch_bounds__(TC2_THREADS, 1)
             if (c.t >= n_ptiles) return;
             const int k = c.kb * TC_K + chunk * 4;
             cf = bl.prep(k, K);
-            if (P > 0) bl.fetch(r, c.p0 + row0, 1, P, k, K);
+            bl.fetch(r, c.p0 + row0, 1, P, k, K);
         };
         auto emit = [&](const Batch4& r, const typename BLoad::Coef& cf, const Cur& c) {
             o3d_mbar_wait(empty + stage, phase ^ 1);
@@ -630,7 +615,7 @@ __global__ void __launch_bounds__(TC2_THREADS, 1)
             uint8_t* xlo = xhi + TILE_BYTES;
 #pragma unroll
             for (int i = 0; i < 4; ++i) {
-                const float4 v = P > 0 ? bl.finish(r, cf, i, c.p0 + row0 + i, P) : make_float4(0.f, 0.f, 0.f, 0.f);
+                const float4 v = bl.finish(r, cf, i, c.p0 + row0 + i, P);
                 const uint32_t off = sw128(row0 + i, chunk);
                 *reinterpret_cast<float4*>(xhi + off) = hi_part(v);
                 *reinterpret_cast<float4*>(xlo + off) = lo_part(v);
@@ -684,59 +669,9 @@ __global__ void __launch_bounds__(TC2_THREADS, 1)
 // SWIZZLE_128B_BASE32B (cute::UMMA::Layout_MN_SW128_32B_Atom): atoms of 4 positions x 32 channels (512 B; one
 // position = one 128-byte row), the 32-byte chunk index XOR-ed with (position % 4).  The producers copy coalesced
 // float4 rows straight into it — no transposition — and the instruction descriptor marks A and B as MN-major.
-//   tile [32 positions x 128 channels]:  atom(cb, pq) at (cb + 4*pq) * 512,  cb = channel/32, pq = position/4
-//   descriptor for k-step ks (8 positions = 2 atoms along K): start = tile + ks*4096,
-//   LBO = 512 (next 32-channel block), SBO = 2048 (next 4 positions)
-constexpr int WG_THREADS = 640;   // warps: 0 MMA | 1 L2 prefetch | 2,3 idle | 4-11 dY producers (4-7 also epilogue) | 12-19 X producers
-constexpr int WG_SMEM = TC_STAGES * STAGE_BYTES + 1024 + 256;
-
-__device__ __forceinline__ uint64_t make_desc_mn(uint32_t smem_addr) {
-    uint64_t d = 0;
-    d |= (uint64_t)((smem_addr >> 4) & 0x3FFF);
-    d |= (uint64_t)(512 >> 4) << 16;    // leading byte offset: between 32-channel blocks
-    d |= (uint64_t)(2048 >> 4) << 32;   // stride byte offset : between 4-position blocks
-    d |= (uint64_t)1 << 46;
-    d |= (uint64_t)1 << 61;             // SWIZZLE_128B_BASE32B
-    return d;
-}
 __host__ __device__ constexpr uint32_t make_idesc_mn(int M, int N) {
     return make_idesc(M, N) | (1u << 15) | (1u << 16);
 }
-__device__ __forceinline__ uint32_t sw128_mn(int p_local, int c4) {   // c4 = float4 index along the 128 channels
-    const int cb = c4 >> 3, c32 = (c4 & 7) >> 1, half = c4 & 1, j0 = p_local & 3;
-    return (uint32_t)((cb + 4 * (p_local >> 2)) * 512 + j0 * 128 + ((c32 ^ j0) << 5) + (half << 4));
-}
-
-// One operand's producer loop of the wgrad kernel: raw loads of k-block kb+1 are issued right after k-block kb has been
-// handed to the tensor core; transform + hi/lo split happen at store time.
-template <class L, class KPos>
-__device__ __forceinline__ void wgrad_produce(const L& ld, uint8_t* smem, int tile_off, uint64_t* full, uint64_t* empty,
-                                              int pt, int c_base, int CH, KPos kpos, int pend, int nkb, int dbg) {
-    const int c4 = pt & 31, prow0 = pt >> 5;      // 256 threads per operand: rows prow0 + 8*i, i < 4
-    const int ch0 = c_base + c4 * 4;
-    const typename L::Coef cf = ld.prep(ch0, CH);
-    typename L::template Batch<4> raw = {};
-    int stage = 0, phase = 0;
-    if (nkb > 0 && !(dbg & 2)) ld.fetch(raw, kpos(0) + prow0, 8, pend, ch0, CH);
-    for (int kb = 0; kb < nkb; ++kb) {
-        o3d_mbar_wait(empty + stage, phase ^ 1);
-        uint8_t* hi = smem + stage * STAGE_BYTES + tile_off;
-        uint8_t* lo = hi + TILE_BYTES;
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const float4 v = ld.finish(raw, cf, i, kpos(kb) + prow0 + 8 * i, pend);
-            const uint32_t off = sw128_mn(prow0 + 8 * i, c4);
-            *reinterpret_cast<float4*>(hi + off) = hi_part(v);
-            *reinterpret_cast<float4*>(lo + off) = lo_part(v);
-        }
-        o3d_fence_proxy_async();
-        o3d_mbar_arrive(full + stage);
-        if (kb + 1 < nkb && !(dbg & 2)) ld.fetch(raw, kpos(kb + 1) + prow0, 8, pend, ch0, CH);
-        if (++stage == TC_STAGES) { stage = 0; phase ^= 1; }
-    }
-}
-
-
 // L2 prefetch of one CTA's slice of position rows, paced by the MMA warp's progress (rows consumed, published in shared
 // memory): at most WINDOW rows ahead.  Prefetching the whole slice up front asks for several hundred MB across the grid —
 // more than the 126 MB L2 — and the lines are evicted again before their k-block comes up (measured: DRAM reads 1.7x the
@@ -757,120 +692,15 @@ __device__ __forceinline__ void paced_prefetch(const LA& da, const LB& xb, int p
     }
 }
 
-template <class XB>
-__global__ void __launch_bounds__(WG_THREADS, 1)
-    pw_wgrad_tc_kernel(TcDy da, XB xb, int P, int M, int N, int chunk, float* __restrict__ dW, int lddw, int dbg) {
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + TC_STAGES * STAGE_BYTES);
-    uint64_t* full = bars;
-    uint64_t* empty = bars + TC_STAGES;
-    uint64_t* tfull = bars + 2 * TC_STAGES;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * TC_STAGES + 1);
-    volatile int* progress = reinterpret_cast<volatile int*>(tmem_slot + 1);   // rows handed to the tensor core so far
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int m0 = blockIdx.z * TC_M, n0 = blockIdx.y * TC_N;
-    // every split owns one contiguous slice of positions (DRAM-friendly; a round-robin deal of k-blocks measured slower)
-    const int pbeg = blockIdx.x * chunk, pend = min(P, pbeg + chunk);
-    const int nkb = pend > pbeg ? (pend - pbeg + TC_K - 1) / TC_K : 0;
-    auto kpos = [&](int i) { return pbeg + i * TC_K; };
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < TC_STAGES; ++s) {
-            o3d_mbar_init(full + s, 512);
-            o3d_mbar_init(empty + s, 1);
-        }
-        o3d_mbar_init(tfull, 1);
-        *progress = 0;
-        o3d_fence_mbar_init();
-    }
-    if (warp == 0) tmem_alloc(tmem_slot, 128);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-
-    if (warp == 0) {
-        const uint32_t idesc = (dbg & 16) ? make_idesc(TC_M, TC_N) : make_idesc_mn(TC_M, TC_N);
-        int stage = 0, phase = 0;
-        for (int kb = 0; kb < nkb; ++kb) {
-            o3d_mbar_wait(full + stage, phase);
-            tc_fence_after();
-            if (lane == 0) {
-                const uint32_t sb = o3d_smem_u32(smem + stage * STAGE_BYTES);
-#pragma unroll
-                for (int pb = 0; pb < TC_K / 8; ++pb) {
-                    const uint32_t o = pb * 4096;
-                    const uint64_t ahi = make_desc_mn(sb + o), alo = make_desc_mn(sb + TILE_BYTES + o);
-                    const uint64_t bhi = make_desc_mn(sb + 2 * TILE_BYTES + o), blo = make_desc_mn(sb + 3 * TILE_BYTES + o);
-                    if (dbg & 32) continue;
-                    umma_tf32(tmem_base, alo, bhi, idesc, (kb | pb) != 0);
-                    umma_tf32(tmem_base, ahi, blo, idesc, 1u);
-                    umma_tf32(tmem_base, ahi, bhi, idesc, 1u);
-                }
-                umma_commit(empty + stage);
-                if (kb == nkb - 1) umma_commit(tfull);
-                *progress = (kb + 1) * TC_K;
-            }
-            __syncwarp();
-            if (++stage == TC_STAGES) { stage = 0; phase ^= 1; }
-        }
-    } else if (warp == 1) {
-        if (lane == 0) {
-            if (dbg & 64) {   // dbg: the old behaviour, whole slice requested up front
-                for (int p = pbeg; p < pend; p += 512) {
-                    da.prefetch_rows(p, 512, pend);
-                    xb.prefetch_rows(p, 512, pend);
-                }
-            } else {
-                paced_prefetch(da, xb, pbeg, pend, progress);
-            }
-        }
-    } else if (warp >= 4) {
-        // producers, 16 warps: 4-11 -> A (dY, channels m0..), 12-19 -> B (X, channels n0..); each thread owns 4 of a
-        // k-block's 32 rows.  (One warp per scheduler and operand could not issue the split + swizzled stores fast enough.)
-        const int pt = (threadIdx.x - 128) & 255;
-        if (warp < 12) wgrad_produce(da, smem, 0, full, empty, pt, m0, M, kpos, pend, nkb, dbg);
-        else wgrad_produce(xb, smem, 2 * TILE_BYTES, full, empty, pt, n0, N, kpos, pend, nkb, dbg);
-        if (warp < 8 && nkb > 0) {   // epilogue: warps 4-7 own TMEM lane quadrants 0-3
-            const int q = warp & 3;
-            const int ch = m0 + q * 32 + lane;
-            o3d_mbar_wait(tfull, 0);
-            tc_fence_after();
-            const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16);
-#pragma unroll 1
-            for (int cg = 0; cg < TC_N / 32; ++cg) {
-                uint32_t r[32];
-                tmem_ld32(taddr + cg * 32, r);
-                if (ch < M) {
-#pragma unroll
-                    for (int j = 0; j < 32; ++j) {
-                        const int n = n0 + cg * 32 + j;
-                        if (n < N) atomicAdd(dW + (size_t)ch * lddw + n, __uint_as_float(r[j]));
-                    }
-                }
-            }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) {
-        tc_fence_after();
-        tmem_dealloc(tmem_base, 128);
-    }
-}
-
-// ------------------------------------------------------------------------------------------------------------
-// wgrad, wide-tile variant: one CTA accumulates a (128*MH) x (128*NH) block of dW (MH*NH accumulators = up to all 512
-// TMEM columns) over its slice of positions, 16 positions per stage.  Relative to the 128x128 kernel above every loaded
-// activation row feeds twice as many MMAs, which halves the L2->SM traffic per FLOP — the limiter of that kernel — and
-// the split-K partial tiles are written with plain coalesced stores into a workspace and summed by a second kernel
-// instead of 65k float REDs per CTA.
+// Wide tiles: one CTA accumulates a (128*MH) x (128*NH) block of dW (MH*NH accumulators = up to all 512 TMEM columns) over
+// its slice of positions, 16 positions per stage.  Against a 128 x 128 tile per CTA with fp32 REDs into dW (the kernel this
+// one replaced) every loaded activation row feeds twice as many MMAs, which halves the L2->SM traffic per FLOP — the limiter
+// of that kernel — and the split-K partial tiles are written with plain coalesced stores into a workspace and summed in a
+// fixed order by a second kernel instead of 65k float REDs per CTA: deterministic, and measured 0.7 % faster over the step.
 //   operand tile [16 positions x 128*H channels], MN-major SWIZZLE_128B_BASE32B: atom(cb, pq) at (cb + 4*H*pq) * 512
 //   descriptor (channel half h, k-step ks): start = tile + h*2048 + ks*2*SBO, LBO = 512, SBO = 4*H*512
 // positions per pipeline stage: each producer thread must keep >= 2 float4 per operand in flight, or the bytes in flight per SM
-// (512 threads x 32 B at 16 positions x 128 channels) cap the kernel near 2.3 TB/s — measured on the 128x128 variant at the SA1
+// (512 threads x 32 B at 16 positions x 128 channels) cap the kernel near 2.3 TB/s — measured on the 128 x 128 kernel at the SA1
 // shapes (ncu, profiles/r2_step_dram_final.txt: 278 us for 629 MB); the single-accumulator variant therefore takes 32 positions
 template <int MH, int NH> constexpr int wg2_k() { return MH * NH == 1 ? 32 : 16; }
 constexpr int WG2_STAGES = 3;
@@ -902,7 +732,7 @@ __device__ __forceinline__ uint32_t sw_mn2(int p_local, int c4) {   // c4 = floa
 
 template <int MH, int NH, class XB>
 __global__ void __launch_bounds__(WG2_THREADS, 1)
-    pw_wgrad_tc2_kernel(TcDy da, XB xb, int P, int M, int N, int chunk, float* __restrict__ part, int dbg) {
+    pw_wgrad_tc2_kernel(TcDy da, XB xb, int P, int M, int N, int chunk, float* __restrict__ part) {
     using C = Wg2Cfg<MH, NH>;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -967,16 +797,7 @@ __global__ void __launch_bounds__(WG2_THREADS, 1)
             if (++stage == WG2_STAGES) { stage = 0; phase ^= 1; }
         }
     } else if (warp == 1) {
-        if (lane == 0) {
-            if (dbg & 64) {
-                for (int p = pbeg; p < pend; p += 512) {
-                    da.prefetch_rows(p, 512, pend);
-                    xb.prefetch_rows(p, 512, pend);
-                }
-            } else {
-                paced_prefetch(da, xb, pbeg, pend, progress);
-            }
-        }
+        if (lane == 0) paced_prefetch(da, xb, pbeg, pend, progress);
     } else {
         // producers (16 warps, 2-17): every thread serves both operands, raw loads first
         const int pt = threadIdx.x - 64;                                // 0..511
@@ -989,7 +810,6 @@ __global__ void __launch_bounds__(WG2_THREADS, 1)
         TcDy::Batch<RA> ra = {};
         typename XB::template Batch<RB> rb = {};
         auto fetch = [&](int kb) {
-            if (dbg & 2) return;
             da.fetch(ra, kpos(kb) + pa0, sa, pend, m0 + ca4 * 4, M);
             xb.fetch(rb, kpos(kb) + pb0, sbs, pend, n0 + cb4 * 4, N);
         };
@@ -1106,16 +926,13 @@ __global__ void w_pretile_kernel(const float* __restrict__ W, int ld, int rows, 
     }
 }
 
-int g_tc_debug = 0, g_tc_force_mt = 0;
-}  // namespace
-extern int o3d_g_fps_wide;
-extern int o3d_g_sa_fused_dbg;
-namespace {
+// o3d_debug_set(0, 1): every tensor-core GEMM takes one 128-channel tile per CTA (MT = 1), for measuring the MT = 2 choice.
+// The library's only mutable global.
+int g_tc_force_mt = 0;
 inline int ilog2_exact(int v) { int l = 0; while ((1 << l) < v) ++l; return l; }
-thread_local int g_tc_rev = 0;   // direction of the next launch (set by the stack sequencer)
 
 template <int MT, class BLoad, class Epi>
-int launch_tc_mt(BLoad bl, const uint8_t* wtiles, int P, int K, int Nw, Epi epi, cudaStream_t st, const char* name) {
+int launch_tc_mt(BLoad bl, const uint8_t* wtiles, int P, int K, int Nw, Epi epi, int rev, cudaStream_t st, const char* name) {
     auto kern = pw_tc_kernel<MT, BLoad, Epi>;
     O3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<MT>::SMEM), name);
     const int mt = (Nw + TC_M - 1) / TC_M;
@@ -1125,7 +942,7 @@ int launch_tc_mt(BLoad bl, const uint8_t* wtiles, int P, int K, int Nw, Epi epi,
     int gx = o3d_num_sms() / gy;
     if (gx < 1) gx = 1;
     if (gx > n_ptiles) gx = n_ptiles;
-    kern<<<dim3(gx, gy), TC2_THREADS, TcCfg<MT>::SMEM, st>>>(bl, wtiles, P, K, Nw, nkb, epi, g_tc_debug, g_tc_rev);
+    kern<<<dim3(gx, gy), TC2_THREADS, TcCfg<MT>::SMEM, st>>>(bl, wtiles, P, K, Nw, nkb, epi, rev);
     O3D_CHECK_LAUNCH(name);
     return O3D_OK;
 }
@@ -1140,12 +957,12 @@ inline bool tc_two_tiles(int Nw, int P = 1 << 30) {
 
 // MTMASK: which MT variants this (loader, epilogue) pair is instantiated for (bit 0: MT = 1, bit 1: MT = 2)
 template <int MTMASK, class BLoad, class Epi>
-int launch_tc(BLoad bl, const uint8_t* wtiles, int P, int K, int Nw, Epi epi, cudaStream_t st, const char* name) {
+int launch_tc(BLoad bl, const uint8_t* wtiles, int P, int K, int Nw, Epi epi, int rev, cudaStream_t st, const char* name) {
     if constexpr ((MTMASK & 2) != 0) {
-        if (tc_two_tiles(Nw, P)) return launch_tc_mt<2>(bl, wtiles, P, K, Nw, epi, st, name);
+        if (tc_two_tiles(Nw, P)) return launch_tc_mt<2>(bl, wtiles, P, K, Nw, epi, rev, st, name);
     }
     if constexpr ((MTMASK & 1) != 0) {
-        if (!tc_two_tiles(Nw, P)) return launch_tc_mt<1>(bl, wtiles, P, K, Nw, epi, st, name);
+        if (!tc_two_tiles(Nw, P)) return launch_tc_mt<1>(bl, wtiles, P, K, Nw, epi, rev, st, name);
     }
     o3d_set_error("%s: no kernel variant for %d output channels", name, Nw);
     return O3D_ERR_ARG;
@@ -1153,13 +970,27 @@ int launch_tc(BLoad bl, const uint8_t* wtiles, int P, int K, int Nw, Epi epi, cu
 
 template <int LD, int MTMASK, class BLoad>
 int launch_fwd(const BLoad& bl, const void* wtiles, const float* bias, int P, int K, int Nw, float* y, int ldy, double* sum,
-               double* sumsq, int S, float* ymax, float* ymin, int32_t* arg, int ldp, cudaStream_t st) {
+               double* sumsq, int S, float* ymax, float* ymin, int32_t* arg, int ldp, int rev, cudaStream_t st) {
     TcFwdEpi<LD> ep{};
     ep.y = y; ep.ldy = ldy; ep.bias = bias; ep.sum = sum; ep.sumsq = sumsq;
     ep.S = S; ep.ymax = ymax; ep.ymin = ymin; ep.arg = arg; ep.ldp = ldp;
     ep.log2S = 0;
     while ((1 << ep.log2S) < S) ++ep.log2S;
-    return launch_tc<MTMASK>(bl, (const uint8_t*)wtiles, P, K, Nw, ep, st, "o3d_pw_fwd_tc");
+    return launch_tc<MTMASK>(bl, (const uint8_t*)wtiles, P, K, Nw, ep, rev, st, "o3d_pw_fwd_tc");
+}
+
+// the usual activation widths get a compile-time row stride (immediate store offsets in the epilogue)
+template <class BLoad>
+int dispatch_fwd(const BLoad& bl, const void* wtiles, const float* bias, int P, int K, int N, float* y, int ldy, double* sum,
+                 double* sumsq, int S, float* ymax, float* ymin, int32_t* arg, int ldp, int rev, cudaStream_t st) {
+    const int Nw = (N + 3) & ~3;
+    const bool two = tc_two_tiles(Nw, P);
+#define O3D_FWD_ARGS bl, wtiles, bias, P, K, Nw, y, ldy, sum, sumsq, S, ymax, ymin, arg, ldp, rev, st
+    if (ldy == 64 && !two) return launch_fwd<64, 1>(O3D_FWD_ARGS);
+    if (ldy == 128 && !two) return launch_fwd<128, 1>(O3D_FWD_ARGS);
+    if (ldy == 256 && two) return launch_fwd<256, 2>(O3D_FWD_ARGS);
+    return launch_fwd<0, 3>(O3D_FWD_ARGS);
+#undef O3D_FWD_ARGS
 }
 
 template <int LD, int MTMASK, bool LIFT = false>
@@ -1174,20 +1005,19 @@ int launch_dgrad(const TcDy& bl, const void* wtiles_t, int P, int Cout, int Cin,
     if (lv) ep.lv = *lv;
     ep.out = out; ep.ldo = ldo; ep.yprev = yprev; ep.ldyp = ldyp; ep.scale = pscale; ep.shift = pshift; ep.relu = prelu;
     ep.s1g = s1; ep.s2y = s2y;
-    // GEMM: D[cin, pos] = sum_cout Wt[cin, cout] * dY[pos, cout]  ->  "K" = Cout, "Nw" = Cin
-    return launch_tc<MTMASK>(bl, (const uint8_t*)wtiles_t, P, Cout, Cin, ep, st, "o3d_pw_dgrad_tc");
+    // GEMM: D[cin, pos] = sum_cout Wt[cin, cout] * dY[pos, cout]  ->  "K" = Cout, "Nw" = Cin; always walks forward
+    return launch_tc<MTMASK>(bl, (const uint8_t*)wtiles_t, P, Cout, Cin, ep, 0, st, "o3d_pw_dgrad_tc");
 }
 
 }  // namespace
 
-extern "C" void o3d_debug_set(int tc_debug, int force_mt) {
-    g_tc_debug = tc_debug;
+extern "C" int o3d_debug_set(int tc_debug, int force_mt) {
+    O3D_REQUIRE(tc_debug == 0 && (force_mt == 0 || force_mt == 1), O3D_ERR_ARG,
+                "o3d_debug_set(%d, %d): tc_debug must be 0 (the profiling switches no longer exist), force_mt 0 or 1", tc_debug,
+                force_mt);
     g_tc_force_mt = force_mt;
-    o3d_g_no_skinny = (tc_debug & 128) != 0;
-    o3d_g_fps_wide = (tc_debug & 1024) != 0;
-    o3d_g_sa_fused_dbg = (tc_debug >> 11) & 15;
+    return O3D_OK;
 }
-extern "C" void o3d_pw_tc_set_reverse(int rev) { g_tc_rev = rev; }
 
 extern "C" long long o3d_pw_tc_wtile_bytes(int rows, int K) {
     const long long mt = (rows + TC_M - 1) / TC_M, nkb = (K + TC_K - 1) / TC_K;
@@ -1204,25 +1034,23 @@ extern "C" int o3d_pw_tc_pretile(const float* w, int ldw, int rows, int K, void*
     return O3D_OK;
 }
 
-extern "C" int o3d_pw_fwd_tc(const float* x, int ldx, const float* in_scale, const float* in_shift, int in_relu,
-                             const void* wtiles, const float* bias, int P, int K, int N, float* y, int ldy, double* sum,
-                             double* sumsq, int S, float* ymax, float* ymin, int32_t* arg, int ldp, void* stream) {
+int pw_fwd_tc(const float* x, int ldx, const float* in_scale, const float* in_shift, int in_relu, const void* wtiles,
+              const float* bias, int P, int K, int N, float* y, int ldy, double* sum, double* sumsq, int S, float* ymax,
+              float* ymin, int32_t* arg, int ldp, int rev, void* stream) {
     O3D_REQUIRE(x && wtiles, O3D_ERR_ARG, "o3d_pw_fwd_tc: null pointer");
     O3D_REQUIRE(P >= 0 && K >= 4 && N >= 1 && (K & 3) == 0 && (ldx & 3) == 0, O3D_ERR_ARG, "o3d_pw_fwd_tc: bad sizes");
     O3D_REQUIRE(S == 0 || (P % S == 0 && 64 % S == 0 && ymax && ymin && arg), O3D_ERR_ARG,
                 "o3d_pw_fwd_tc: pooling group size must divide 64 and P");
     if (P == 0) return O3D_OK;
-    const int Nw = (N + 3) & ~3;
-    TcAct bl{x, ldx, in_scale, in_shift, in_relu};
-    // the usual activation widths get a compile-time row stride (immediate store offsets in the epilogue)
-    cudaStream_t st = (cudaStream_t)stream;
-    const bool two = tc_two_tiles(Nw, P);
-#define O3D_FWD_ARGS bl, wtiles, bias, P, K, Nw, y, ldy, sum, sumsq, S, ymax, ymin, arg, ldp, st
-    if (ldy == 64 && !two) return launch_fwd<64, 1>(O3D_FWD_ARGS);
-    if (ldy == 128 && !two) return launch_fwd<128, 1>(O3D_FWD_ARGS);
-    if (ldy == 256 && two) return launch_fwd<256, 2>(O3D_FWD_ARGS);
-    return launch_fwd<0, 3>(O3D_FWD_ARGS);
-#undef O3D_FWD_ARGS
+    const TcAct bl{x, ldx, in_scale, in_shift, in_relu};
+    return dispatch_fwd(bl, wtiles, bias, P, K, N, y, ldy, sum, sumsq, S, ymax, ymin, arg, ldp, rev, (cudaStream_t)stream);
+}
+
+extern "C" int o3d_pw_fwd_tc(const float* x, int ldx, const float* in_scale, const float* in_shift, int in_relu,
+                             const void* wtiles, const float* bias, int P, int K, int N, float* y, int ldy, double* sum,
+                             double* sumsq, int S, float* ymax, float* ymin, int32_t* arg, int ldp, void* stream) {
+    return pw_fwd_tc(x, ldx, in_scale, in_shift, in_relu, wtiles, bias, P, K, N, y, ldy, sum, sumsq, S, ymax, ymin, arg, ldp, 0,
+                     stream);
 }
 
 namespace {
@@ -1233,7 +1061,7 @@ int dgrad_tc_impl(const float* g, int ldg, const float* y, int ldy, const float*
     O3D_REQUIRE((g || dpool) && wtiles_t && out, O3D_ERR_ARG, "o3d_pw_dgrad_tc: null pointer");
     O3D_REQUIRE((Cout & 3) == 0 && (Cin & 3) == 0, O3D_ERR_ARG, "o3d_pw_dgrad_tc: channel counts must be multiples of 4");
     if (P == 0) return O3D_OK;
-    TcDy bl{g, ldg, y, ldy, a, b, cc, dpool, sel, S > 0 ? S : 1, ldp, ilog2_exact(S > 0 ? S : 1), g_tc_debug};
+    TcDy bl{g, ldg, y, ldy, a, b, cc, dpool, sel, S > 0 ? S : 1, ldp, ilog2_exact(S > 0 ? S : 1)};
     cudaStream_t st = (cudaStream_t)stream;
     const bool two = tc_two_tiles(Cin, P);
     const int ld = (!yprev || ldyp == ldo) ? ldo : 0;   // one compile-time stride serves both out and yprev
@@ -1253,51 +1081,6 @@ extern "C" int o3d_pw_dgrad_tc(const float* g, int ldg, const float* y, int ldy,
                                void* stream) {
     return dgrad_tc_impl(g, ldg, y, ldy, a, b, cc, dpool, sel, S, ldp, wtiles_t, P, Cout, Cin, out, ldo, yprev, ldyp, pscale,
                          pshift, prelu, s1, s2y, stream, nullptr);
-}
-
-// dgrad whose input side is a lifted first layer: the ReLU mask and the BatchNorm-backward sums use Y0 gathered from Z
-extern "C" int o3d_pw_dgrad_tc_lift(const float* g, int ldg, const float* y, int ldy, const float* a, const float* b,
-                                    const float* cc, const float* dpool, const int32_t* sel, int S, int ldp,
-                                    const void* wtiles_t, int P, int Cout, int Cin, float* out, int ldo,
-                                    const o3d_lift_t* lf, const int32_t* gidx, const float* pscale, const float* pshift,
-                                    int prelu, double* s1, double* s2y, void* stream) {
-    O3D_REQUIRE(lf && (gidx || !lf->z) && (lf->z || lf->s) && lf->ldz == Cin, O3D_ERR_ARG, "o3d_pw_dgrad_tc_lift: lift descriptor");
-    const LiftView lv{lf->z, lf->ldz, lf->z ? gidx : nullptr, lf->s, lf->u};
-    return dgrad_tc_impl(g, ldg, y, ldy, a, b, cc, dpool, sel, S, ldp, wtiles_t, P, Cout, Cin, out, ldo, nullptr, 0, pscale,
-                         pshift, prelu, s1, s2y, stream, &lv);
-}
-
-namespace {
-template <class XB>
-int launch_wgrad1(const TcDy& da, const XB& xb, int P, int Cout, int Cin, float* dw, int lddw, cudaStream_t st) {
-    auto kern = pw_wgrad_tc_kernel<XB>;
-    O3D_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, WG_SMEM), "o3d_pw_wgrad_tc");
-    const int mt = (Cout + TC_M - 1) / TC_M, nt = (Cin + TC_N - 1) / TC_N;
-    int splits = o3d_num_sms() / (mt * nt);
-    if (splits < 1) splits = 1;
-    int chunk = (P + splits - 1) / splits;
-    chunk = ((chunk + TC_K - 1) / TC_K) * TC_K;
-    splits = (P + chunk - 1) / chunk;
-    kern<<<dim3(splits, nt, mt), WG_THREADS, WG_SMEM, st>>>(da, xb, P, Cout, Cin, chunk, dw, lddw, g_tc_debug);
-    O3D_CHECK_LAUNCH("o3d_pw_wgrad_tc");
-    return O3D_OK;
-}
-inline TcLift make_tclift(const o3d_lift_t* lf, const int32_t* gidx, const float* scale, const float* shift, int relu) {
-    return TcLift{LiftView{lf->z, lf->ldz, lf->z ? gidx : nullptr, lf->s, lf->u}, scale, shift, relu, 0};
-}
-}  // namespace
-
-extern "C" int o3d_pw_wgrad_tc(const float* g, int ldg, const float* y, int ldy, const float* a, const float* b,
-                               const float* cc, const float* dpool, const int32_t* sel, int S, int ldp, const float* x,
-                               int ldx, const float* in_scale, const float* in_shift, int in_relu, int P, int Cout,
-                               int Cin, float* dw, int lddw, void* stream) {
-    O3D_REQUIRE((g || dpool) && x && dw, O3D_ERR_ARG, "o3d_pw_wgrad_tc: null pointer");
-    O3D_REQUIRE((Cout & 3) == 0 && (Cin & 3) == 0 && (ldx & 3) == 0, O3D_ERR_ARG,
-                "o3d_pw_wgrad_tc: channel counts / leading dimensions must be multiples of 4");
-    if (P == 0) return O3D_OK;
-    TcDy da{g, ldg, y, ldy, a, b, cc, dpool, sel, S > 0 ? S : 1, ldp, ilog2_exact(S > 0 ? S : 1), g_tc_debug};
-    TcAct xb{x, ldx, in_scale, in_shift, in_relu};
-    return launch_wgrad1(da, xb, P, Cout, Cin, dw, lddw, (cudaStream_t)stream);
 }
 
 namespace {
@@ -1323,7 +1106,7 @@ int launch_wgrad2(const TcDy& da, const XB& xb, int P, int Cout, int Cin, float*
     int chunk = (P + splits - 1) / splits;
     chunk = ((chunk + C::K - 1) / C::K) * C::K;
     splits = (P + chunk - 1) / chunk;
-    kern<<<dim3(splits, nt, mt), WG2_THREADS, C::SMEM, st>>>(da, xb, P, Cout, Cin, chunk, part, g_tc_debug);
+    kern<<<dim3(splits, nt, mt), WG2_THREADS, C::SMEM, st>>>(da, xb, P, Cout, Cin, chunk, part);
     O3D_CHECK_LAUNCH("o3d_pw_wgrad_tc2");
     dim3 rg((Cin / 4 + 31) / 32, Cout);
     wgrad_reduce_kernel<<<rg, 256, 0, st>>>(part, splits, Mt, Nt, Cout, Cin, dw, lddw);
@@ -1339,6 +1122,9 @@ int dispatch_wgrad2(const TcDy& da, const XB& xb, int P, int Cout, int Cin, floa
     if (n2) return launch_wgrad2<1, 2>(da, xb, P, Cout, Cin, dw, lddw, part, part_floats, st);
     return launch_wgrad2<1, 1>(da, xb, P, Cout, Cin, dw, lddw, part, part_floats, st);
 }
+inline TcLift make_tclift(const o3d_lift_t* lf, const int32_t* gidx, const float* scale, const float* shift, int relu) {
+    return TcLift{LiftView{lf->z, lf->ldz, lf->z ? gidx : nullptr, lf->s, lf->u}, scale, shift, relu, 0};
+}
 }  // namespace
 
 extern "C" long long o3d_pw_wgrad_tc2_workspace_floats(void) {
@@ -1353,45 +1139,45 @@ extern "C" int o3d_pw_wgrad_tc2(const float* g, int ldg, const float* y, int ldy
     O3D_REQUIRE((Cout & 3) == 0 && (Cin & 3) == 0 && (ldx & 3) == 0 && (lddw & 3) == 0, O3D_ERR_ARG,
                 "o3d_pw_wgrad_tc2: channel counts / leading dimensions must be multiples of 4");
     if (P == 0) return O3D_OK;
-    TcDy da{g, ldg, y, ldy, a, b, cc, dpool, sel, S > 0 ? S : 1, ldp, ilog2_exact(S > 0 ? S : 1), g_tc_debug};
+    TcDy da{g, ldg, y, ldy, a, b, cc, dpool, sel, S > 0 ? S : 1, ldp, ilog2_exact(S > 0 ? S : 1)};
     TcAct xb{x, ldx, in_scale, in_shift, in_relu};
     return dispatch_wgrad2(da, xb, P, Cout, Cin, dw, lddw, part, part_floats, (cudaStream_t)stream);
 }
 
 // ---- lifted first layer (o3d_lift_t): the next layer's GEMMs read Y0 through TcLift / the lifted dgrad epilogue ----------
-extern "C" int o3d_pw_wgrad_tc_lift(const float* g, int ldg, const float* y, int ldy, const float* a, const float* b,
-                                    const float* cc, const float* dpool, const int32_t* sel, int S, int ldp,
-                                    const o3d_lift_t* lf, const int32_t* gidx, const float* in_scale, const float* in_shift,
-                                    int in_relu, int P, int Cout, int Cin, float* dw, int lddw, float* part,
-                                    long long part_floats, void* stream) {
-    O3D_REQUIRE((g || dpool) && lf && (gidx || !lf->z) && dw, O3D_ERR_ARG, "o3d_pw_wgrad_tc_lift: null pointer");
-    O3D_REQUIRE((Cout & 3) == 0 && (Cin & 3) == 0 && lf->ldz == Cin && (lddw & 3) == 0, O3D_ERR_ARG,
-                "o3d_pw_wgrad_tc_lift: channel counts / leading dimensions");
+int pw_fwd_tc_lift(const o3d_lift_t* lf, const int32_t* gidx, const float* in_scale, const float* in_shift, int in_relu,
+                   const void* wtiles, const float* bias, int P, int K, int N, float* y, int ldy, double* sum, double* sumsq,
+                   int S, float* ymax, float* ymin, int32_t* arg, int ldp, int rev, void* stream) {
+    O3D_REQUIRE(lf && (gidx || !lf->z) && wtiles, O3D_ERR_ARG, "pw_fwd_tc_lift: null pointer");
+    O3D_REQUIRE(P >= 0 && K >= 32 && N >= 1 && (K & 3) == 0 && lf->ldz == K, O3D_ERR_ARG, "pw_fwd_tc_lift: bad sizes");
+    O3D_REQUIRE(S == 0 || (P % S == 0 && 64 % S == 0 && ymax && ymin && arg), O3D_ERR_ARG,
+                "pw_fwd_tc_lift: pooling group size must divide 64 and P");
     if (P == 0) return O3D_OK;
-    TcDy da{g, ldg, y, ldy, a, b, cc, dpool, sel, S > 0 ? S : 1, ldp, ilog2_exact(S > 0 ? S : 1), g_tc_debug};
-    TcLift xb = make_tclift(lf, gidx, in_scale, in_shift, in_relu);
-    xb.la = part ? ((Cout > 128 || Cin > 128) ? 16 : 32) : TC_K;      // a producer thread's next fetch lies one k-block of positions further
-    if (part) return dispatch_wgrad2(da, xb, P, Cout, Cin, dw, lddw, part, part_floats, (cudaStream_t)stream);
-    return launch_wgrad1(da, xb, P, Cout, Cin, dw, lddw, (cudaStream_t)stream);
+    const TcLift bl = make_tclift(lf, gidx, in_scale, in_shift, in_relu);
+    return dispatch_fwd(bl, wtiles, bias, P, K, N, y, ldy, sum, sumsq, S, ymax, ymin, arg, ldp, rev, (cudaStream_t)stream);
 }
 
-extern "C" int o3d_pw_fwd_tc_lift(const o3d_lift_t* lf, const int32_t* gidx, const float* in_scale, const float* in_shift,
-                                  int in_relu, const void* wtiles, const float* bias, int P, int K, int N, float* y, int ldy,
-                                  double* sum, double* sumsq, int S, float* ymax, float* ymin, int32_t* arg, int ldp,
-                                  void* stream) {
-    O3D_REQUIRE(lf && (gidx || !lf->z) && wtiles, O3D_ERR_ARG, "o3d_pw_fwd_tc_lift: null pointer");
-    O3D_REQUIRE(P >= 0 && K >= 32 && N >= 1 && (K & 3) == 0 && lf->ldz == K, O3D_ERR_ARG, "o3d_pw_fwd_tc_lift: bad sizes");
-    O3D_REQUIRE(S == 0 || (P % S == 0 && 64 % S == 0 && ymax && ymin && arg), O3D_ERR_ARG,
-                "o3d_pw_fwd_tc_lift: pooling group size must divide 64 and P");
+// dgrad whose input side is a lifted first layer: the ReLU mask and the BatchNorm-backward sums use Y0 gathered from Z
+int pw_dgrad_tc_lift(const float* g, int ldg, const float* y, int ldy, const float* a, const float* b, const float* cc,
+                     const float* dpool, const int32_t* sel, int S, int ldp, const void* wtiles_t, int P, int Cout, int Cin,
+                     float* out, int ldo, const o3d_lift_t* lf, const int32_t* gidx, const float* pscale, const float* pshift,
+                     int prelu, double* s1, double* s2y, void* stream) {
+    O3D_REQUIRE(lf && (gidx || !lf->z) && (lf->z || lf->s) && lf->ldz == Cin, O3D_ERR_ARG, "pw_dgrad_tc_lift: lift descriptor");
+    const LiftView lv{lf->z, lf->ldz, lf->z ? gidx : nullptr, lf->s, lf->u};
+    return dgrad_tc_impl(g, ldg, y, ldy, a, b, cc, dpool, sel, S, ldp, wtiles_t, P, Cout, Cin, out, ldo, nullptr, 0, pscale,
+                         pshift, prelu, s1, s2y, stream, &lv);
+}
+
+int pw_wgrad_tc_lift(const float* g, int ldg, const float* y, int ldy, const float* a, const float* b, const float* cc,
+                     const float* dpool, const int32_t* sel, int S, int ldp, const o3d_lift_t* lf, const int32_t* gidx,
+                     const float* in_scale, const float* in_shift, int in_relu, int P, int Cout, int Cin, float* dw, int lddw,
+                     float* part, long long part_floats, void* stream) {
+    O3D_REQUIRE((g || dpool) && lf && (gidx || !lf->z) && dw && part, O3D_ERR_ARG, "pw_wgrad_tc_lift: null pointer");
+    O3D_REQUIRE((Cout & 3) == 0 && (Cin & 3) == 0 && lf->ldz == Cin && (lddw & 3) == 0, O3D_ERR_ARG,
+                "pw_wgrad_tc_lift: channel counts / leading dimensions");
     if (P == 0) return O3D_OK;
-    const int Nw = (N + 3) & ~3;
-    const TcLift bl = make_tclift(lf, gidx, in_scale, in_shift, in_relu);
-    cudaStream_t st = (cudaStream_t)stream;
-    const bool two = tc_two_tiles(Nw, P);
-#define O3D_FWD_ARGS bl, wtiles, bias, P, K, Nw, y, ldy, sum, sumsq, S, ymax, ymin, arg, ldp, st
-    if (ldy == 64 && !two) return launch_fwd<64, 1>(O3D_FWD_ARGS);
-    if (ldy == 128 && !two) return launch_fwd<128, 1>(O3D_FWD_ARGS);
-    if (ldy == 256 && two) return launch_fwd<256, 2>(O3D_FWD_ARGS);
-    return launch_fwd<0, 3>(O3D_FWD_ARGS);
-#undef O3D_FWD_ARGS
+    TcDy da{g, ldg, y, ldy, a, b, cc, dpool, sel, S > 0 ? S : 1, ldp, ilog2_exact(S > 0 ? S : 1)};
+    TcLift xb = make_tclift(lf, gidx, in_scale, in_shift, in_relu);
+    xb.la = (Cout > 128 || Cin > 128) ? 16 : 32;      // a producer thread's next fetch lies one k-block of positions further
+    return dispatch_wgrad2(da, xb, P, Cout, Cin, dw, lddw, part, part_floats, (cudaStream_t)stream);
 }

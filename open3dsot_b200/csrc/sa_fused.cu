@@ -29,8 +29,6 @@
 #include "tc_ptx.cuh"
 #include "../../include/o3d_b200.h"
 
-int o3d_g_sa_fused_dbg = 0;   // experiments (o3d_debug_set bits 11-14): 1 = every weight tile as 4 bulk copies; wrong results: 2 = no weight copies, 4 = no MMAs, 8 = no epilogue work
-
 namespace {
 
 constexpr int SF_POS = 64;                  // positions per CTA
@@ -59,7 +57,7 @@ struct SfParams {
     int n, Cp, ldf, N, M, S, BM;
     float radius, radius2;
     int normalize;
-    int act_bytes, nslot, dbg;
+    int act_bytes, nslot;
     uint32_t wx_off;       // floats: W0's coordinate columns, [3][n_mt0 * 128]
     uint32_t tiles_off;    // bytes: weight tiles in consumption order (layer, channel tile, k-block)
     SfLayer l[O3D_MAX_LAYERS];
@@ -123,7 +121,6 @@ __global__ void __launch_bounds__(SF_THREADS, 2)
                         const uint32_t d_tmem = tmem_base + (uint32_t)(mt * SF_POS);
 #pragma unroll
                         for (int ks = 0; ks < TC_K / 8; ++ks) {
-                            if (prm.dbg & 4) break;
                             const uint64_t adv = (uint64_t)((ks * 32) >> 4);   // +32 bytes along K inside the 128-byte swizzle row
                             umma_tf32(d_tmem, wlo + adv, xhi + adv, idesc, (kb | ks) != 0);
                             umma_tf32(d_tmem, whi + adv, xlo + adv, idesc, 1u);
@@ -147,17 +144,8 @@ __global__ void __launch_bounds__(SF_THREADS, 2)
                 if (!L.mma) continue;
                 for (int t = 0; t < L.n_mt * L.nkb; ++t) {
                     o3d_mbar_wait(empty + slot, phase ^ 1);
-                    if (prm.dbg & 2) {
-                        o3d_mbar_arrive(full + slot);
-                    } else if (prm.dbg & 1) {
-                        o3d_mbar_expect_tx(full + slot, SF_WTILE);
-#pragma unroll
-                        for (int c = 0; c < 4; ++c)
-                            o3d_bulk_g2s(ring + slot * SF_WTILE + c * (SF_WTILE / 4), src + c * (SF_WTILE / 4), SF_WTILE / 4, full + slot);
-                    } else {
-                        o3d_mbar_expect_tx(full + slot, SF_WTILE);
-                        o3d_bulk_g2s(ring + slot * SF_WTILE, src, SF_WTILE, full + slot);
-                    }
+                    o3d_mbar_expect_tx(full + slot, SF_WTILE);
+                    o3d_bulk_g2s(ring + slot * SF_WTILE, src, SF_WTILE, full + slot);
                     src += SF_WTILE;
                     if (++slot == nslot) { slot = 0; phase ^= 1; }
                 }
@@ -254,7 +242,7 @@ __global__ void __launch_bounds__(SF_THREADS, 2)
             const int m = wide ? half : 0;
             const int kb_out = m * 4 + q;               // the k-block of the next operand this warp's 32 channels form
             // channels past the layer's width are padding: nothing reads them
-            const bool work = (wide || S <= 32 || half == 0) && (last ? kb_out * 32 < L.cout : kb_out < prm.l[l + 1].nkb) && !(prm.dbg & 8);
+            const bool work = (wide || S <= 32 || half == 0) && (last ? kb_out * 32 < L.cout : kb_out < prm.l[l + 1].nkb);
             const int col0 = all_cols ? 0 : half * 32, ncol = all_cols ? 64 : 32;
             const int chl = kb_out * 32 + lane;         // this thread's output channel
             float sc = 0.f, sh = 0.f, wx0 = 0.f, wx1 = 0.f, wx2 = 0.f;
@@ -502,7 +490,6 @@ extern "C" int o3d_sa_fused_forward(const o3d_stack_t* d, const void* block, con
         if (fit >= 2 && fit < nslot) nslot = fit;
     }
     prm.nslot = nslot;
-    prm.dbg = o3d_g_sa_fused_dbg;
     const int smem = 1024 + act + nslot * SF_WTILE + SF_MISC;
     O3D_CUDA(cudaFuncSetAttribute(sa_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem), "o3d_sa_fused_forward: smem attribute");
     sa_fused_kernel<<<grid, SF_THREADS, smem, (cudaStream_t)stream>>>(prm, (const uint8_t*)block, xyz, new_xyz, feat_cl, out, ldo, idx);

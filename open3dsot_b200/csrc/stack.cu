@@ -9,6 +9,7 @@
 // stack can be captured into a CUDA graph.
 #include <string.h>
 #include "common.cuh"
+#include "pwmlp_tc.cuh"
 #include "../../include/o3d_b200.h"
 
 namespace {
@@ -139,7 +140,7 @@ struct Plan {
 };
 
 bool make_plan(const o3d_stack_t* d, Plan& p) {
-    if (d->n_layers < 1 || d->n_layers > O3D_MAX_LAYERS || d->P < 0 || d->K0 < 4 || (d->K0 & 3)) return false;
+    if (d->n_layers < 1 || d->n_layers > O3D_MAX_LAYERS || d->P < 0 || d->K0 < 4 || (d->K0 & 3) || (d->use_tc & ~3)) return false;
     p.n = d->n_layers; p.P = d->P; p.S = d->S;
     p.rows = d->S > 0 ? d->P / d->S : d->P;
     p.lift = d->lift != nullptr;
@@ -162,7 +163,7 @@ bool make_plan(const o3d_stack_t* d, Plan& p) {
         // Y0 stays virtual when all three GEMMs of layer 1 run on the tensor cores over whole 32-channel k-blocks
         const bool tcw1 = (d->use_tc & 2) && p.Nw[1] >= 64 && p.K[1] >= 64 && d->P >= 4096;
         // (inference: no weight-gradient kernel will run, so its size floor P >= 4096 does not apply)
-        p.virt = p.tc_f[1] && p.tc_b[1] && (tcw1 || !d->training) && tc_main(p.K[1]) == p.K[1] && p.K[1] % 32 == 0 && !(d->use_tc & 8);
+        p.virt = p.tc_f[1] && p.tc_b[1] && (tcw1 || !d->training) && tc_main(p.K[1]) == p.K[1] && p.K[1] % 32 == 0;
     }
     // statistics block first (one memset)
     p.stat_all = o;
@@ -327,15 +328,13 @@ extern "C" int o3d_stack_forward(const o3d_stack_t* d, const float* x, void* ws_
             // lifted layer: one gather pass = row indices + batch statistics (+ Y0 itself on the CUDA-core fallback)
             rc = o3d_lift_stats(d->lift, p.P, Nw, at<int32_t>(ws, p.gidx), p.virt ? nullptr : y, sum, sumsq, stream);
         } else if (l == 1 && p.virt) {
-            o3d_pw_tc_set_reverse(0);
-            rc = o3d_pw_fwd_tc_lift(d->lift, at<int32_t>(ws, p.gidx), in_scale, in_shift, in_relu, wsp + p.tiles[l], bias, p.P, K,
-                                    cout, y, Nw, sum, sumsq, pool ? p.S : 0, ymax, ymin, arg, Nw, stream);
+            rc = pw_fwd_tc_lift(d->lift, at<int32_t>(ws, p.gidx), in_scale, in_shift, in_relu, wsp + p.tiles[l], bias, p.P, K, cout,
+                                y, Nw, sum, sumsq, pool ? p.S : 0, ymax, ymin, arg, Nw, 0, stream);
         } else if (p.tc_f[l]) {
             // snake order: layer 0 starts where the grouping kernel finished (the end), layer 1 where layer 0 finished, ...
-            o3d_pw_tc_set_reverse((l & 1) == 0);
             void* tiles = wsp + p.tiles[l];
-            rc = o3d_pw_fwd_tc(cur, cur_ld, in_scale, in_shift, in_relu, tiles, bias, p.P, K, cout, y, Nw, sum, sumsq,
-                               pool ? p.S : 0, ymax, ymin, arg, Nw, stream);
+            rc = pw_fwd_tc(cur, cur_ld, in_scale, in_shift, in_relu, tiles, bias, p.P, K, cout, y, Nw, sum, sumsq, pool ? p.S : 0,
+                           ymax, ymin, arg, Nw, (l & 1) == 0, stream);
         } else {
             rc = o3d_pw_fwd(cur, cur_ld, in_scale, in_shift, in_relu, wt, Nw, bias, p.P, K, cout, y, Nw, sum, sumsq,
                             pool ? p.S : 0, ymax, ymin, arg, Nw, stream);
@@ -452,11 +451,9 @@ extern "C" int o3d_stack_backward(const o3d_stack_t* d, const float* x, const vo
             double* ps1 = want ? s1(l - 1) : nullptr;
             double* ps2 = want ? s1(l - 1) + K : nullptr;
             if (l == 1 && p.virt) {
-                o3d_pw_tc_set_reverse(0);
-                rc = o3d_pw_dgrad_tc_lift(gl, Nl, yl, Nl, a, b, cc, dpl, sel, Sg, Nl, wf + p.btiles[l], p.P, Nl, K, gout, K, d->lift,
-                                          at<int32_t>(wf, p.gidx), psc, psh, prelu, ps1, ps2, stream);
+                rc = pw_dgrad_tc_lift(gl, Nl, yl, Nl, a, b, cc, dpl, sel, Sg, Nl, wf + p.btiles[l], p.P, Nl, K, gout, K, d->lift,
+                                      at<int32_t>(wf, p.gidx), psc, psh, prelu, ps1, ps2, stream);
             } else if (p.tc_b[l]) {
-                o3d_pw_tc_set_reverse(0);   // dgrad sweeps forward; the wgrad that follows sweeps the same rows backward
                 // tensor cores on the first floor(K/128)*128 input channels, exact CUDA-core kernel on the ragged tail
                 // (the xyz / box-cloud extras of a first layer)
                 const int Km = tc_main(K);
@@ -481,23 +478,17 @@ extern "C" int o3d_stack_backward(const o3d_stack_t* d, const float* x, const vo
         if (d->d_weight[l]) {
             float* dwp = at<float>(wb, p.dwp[l]);
             const bool tcw = (d->use_tc & 2) && Nl >= 64 && K >= 64 && p.P >= 4096;
+            // every tensor-core weight gradient goes through the split-K kernel whose partial tiles are summed by a second kernel
+            // in a fixed order (deterministic)
             if (l == 1 && p.virt) {
-                // every tensor-core weight gradient goes through the split-K kernel whose partial tiles are summed by a second
-                // kernel in a fixed order (deterministic; measured 0.7 % faster over the step than the fp32-RED 128x128 kernel,
-                // which use_tc bit 2 still selects)
-                const bool wide = (d->use_tc & 4) == 0;
-                rc = o3d_pw_wgrad_tc_lift(gl, Nl, yl, Nl, a, b, cc, dpl, sel, Sg, Nl, d->lift, at<int32_t>(wf, p.gidx), psc, psh, prelu,
-                                          p.P, Nl, K, dwp, K, wide ? at<float>(wb, p.wpart) : nullptr, p.wpart_floats, stream);
+                rc = pw_wgrad_tc_lift(gl, Nl, yl, Nl, a, b, cc, dpl, sel, Sg, Nl, d->lift, at<int32_t>(wf, p.gidx), psc, psh, prelu, p.P,
+                                      Nl, K, dwp, K, at<float>(wb, p.wpart), p.wpart_floats, stream);
             } else if (tcw) {
                 // tensor-core part: the first floor(K/128)*128 input channels; ragged tail (xyz / box-cloud extras)
                 // goes through the exact CUDA-core kernel on the remaining columns
                 const int Kmain = tc_main(K);
-                if ((d->use_tc & 4) == 0)       // deterministic split-K + ordered reduction (see above); bit 2: fp32-RED kernel
-                    rc = o3d_pw_wgrad_tc2(gl, Nl, yl, Nl, a, b, cc, dpl, sel, Sg, Nl, xin, K, psc, psh, prelu, p.P, Nl, Kmain, dwp,
-                                          K, at<float>(wb, p.wpart), p.wpart_floats, stream);
-                else
-                    rc = o3d_pw_wgrad_tc(gl, Nl, yl, Nl, a, b, cc, dpl, sel, Sg, Nl, xin, K, psc, psh, prelu, p.P, Nl, Kmain, dwp,
-                                         K, stream);
+                rc = o3d_pw_wgrad_tc2(gl, Nl, yl, Nl, a, b, cc, dpl, sel, Sg, Nl, xin, K, psc, psh, prelu, p.P, Nl, Kmain, dwp, K,
+                                      at<float>(wb, p.wpart), p.wpart_floats, stream);
                 if (rc) return rc;
                 if (K > Kmain)
                     rc = o3d_pw_wgrad(gl, Nl, yl, Nl, a, b, cc, dpl, sel, Sg, Nl, xin + Kmain, K, psc ? psc + Kmain : nullptr,

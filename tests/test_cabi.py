@@ -90,3 +90,24 @@ def test_fused_sa_layer_plan_and_argument_checks():
     assert b"features" in L.o3d_last_error()
     assert L.o3d_resample(16, 16, 16, 16, 1, 100, 4096, 16, 16, 16, None, None) < 0        # size > 2048
     assert b"size" in L.o3d_last_error()
+
+
+def test_stack_plan_rejects_unknown_use_tc_bits():
+    """use_tc has two bits (tensor-core forward + dgrad, tensor-core wgrad); a descriptor with any other bit set is refused
+    instead of silently running the default kernels"""
+    L = _lib.lib()
+    d = _sa_desc(64, [128, 128])
+    d.P, d.S, d.training = 256, 32, 1
+    for use_tc, ok in ((3, True), (7, False), (11, False)):
+        d.use_tc = use_tc
+        for backward in (0, 1):
+            n = L.o3d_stack_workspace_bytes(ctypes.byref(d), backward)
+            assert (n > 0) if ok else (n == -1), (use_tc, backward, n)
+
+
+def test_debug_set_accepts_only_the_force_mt_switch():
+    L = _lib.lib()
+    assert L.o3d_debug_set(1, 0) < 0
+    assert b"o3d_debug_set" in L.o3d_last_error()
+    assert L.o3d_debug_set(0, 2) < 0
+    assert L.o3d_debug_set(0, 0) == 0

@@ -30,13 +30,9 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--batch", type=int, default=48)
     ap.add_argument("--iters", type=int, default=10)
-    ap.add_argument("--dbg", type=int, default=0, help="o3d_debug_set value (1024 = wide FPS variant)")
     a = ap.parse_args()
     dev = torch.device("cuda", 0)
     B = a.batch
-    if a.dbg:
-        from open3dsot_b200 import _lib
-        _lib.lib().o3d_debug_set(a.dbg, 0)
     b = synthetic_siamese_batch(B, 512, 1024, seed=20260924)
     search = b["search_points"].to(dev)
     tmpl = b["template_points"].to(dev)

@@ -61,11 +61,7 @@ def main():
     ap.add_argument("--iters", type=int, default=20)
     ap.add_argument("--only-fused", action="store_true")
     ap.add_argument("--eager", action="store_true", help="no CUDA graph (for ncu)")
-    ap.add_argument("--dbg", type=int, default=0, help="o3d_debug_set value (2048: 4 bulk copies per weight tile, 4096: no weight copies)")
     a = ap.parse_args()
-    if a.dbg:
-        from open3dsot_b200 import _lib
-        _lib.lib().o3d_debug_set(a.dbg, 0)
     torch.manual_seed(0)
     res = {}
     with torch.no_grad(), runtime.static_weights_scope():

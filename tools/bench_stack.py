@@ -24,7 +24,6 @@ def main():
     ap.add_argument("--levels", default="0,1,3")
     ap.add_argument("--iters", type=int, default=10)
     ap.add_argument("--fwd-only", action="store_true")
-    ap.add_argument("--dbg", default="0", help="comma-separated o3d_debug_set values, one measurement per value")
     ap.add_argument("--profile", action="store_true", help="print per-kernel device times of one fwd+bwd (CUPTI)")
     ap.add_argument("--no-dx", action="store_true", help="the stack input needs no gradient (first SA level)")
     ap.add_argument("--force-mt", type=int, default=0)
@@ -41,8 +40,8 @@ def main():
     fwd_fl = sum(nw[i] + nw[i + 1] for i in range(len(nw) - 1))
     bwd_fl = sum(2 * nw[i + 1] + 2 * nw[i] for i in range(len(nw) - 1)) + sum(2 * nw[i + 1] + nw[i] for i in range(len(nw) - 1))
     gb_f, gb_b = 4e-9 * P * fwd_fl, 4e-9 * P * bwd_fl
-    for lv, dbg in [(int(v), int(d)) for v in a.levels.split(",") for d in a.dbg.split(",")]:
-        _lib.lib().o3d_debug_set(dbg, a.force_mt)
+    _lib.check(_lib.lib().o3d_debug_set(0, a.force_mt), "o3d_debug_set")
+    for lv in [int(v) for v in a.levels.split(",")]:
         runtime.set_tc(lv)
         xin = x.clone().requires_grad_(not a.fwd_only and not a.no_dx)
         for _ in range(2):
@@ -78,7 +77,7 @@ def main():
             for e in evs[2 * n:]:
                 if e.device_time > 8:
                     print(f"    {e.device_time:9.1f} us  {e.name[:110]}")
-        print(f"shape {a.shape} P={P} level {lv} dbg {dbg}: fwd {tf:.3f} ms ({flops / tf / 1e9:.1f} TFLOP/s, {gb_f / tf * 1e3:.0f} GB/s)"
+        print(f"shape {a.shape} P={P} level {lv}: fwd {tf:.3f} ms ({flops / tf / 1e9:.1f} TFLOP/s, {gb_f / tf * 1e3:.0f} GB/s)"
               f"  bwd {tb:.3f} ms ({2 * flops / max(tb, 1e-9) / 1e9:.1f} TFLOP/s, {gb_b / max(tb, 1e-9) * 1e3:.0f} GB/s)", flush=True)
 
 
